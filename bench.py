@@ -4,6 +4,7 @@ steps, CFG 3.5, fp16).
 
     python bench.py --gpus N --steps K --warmup W             # product arm (sm_100a kernels)
     python bench.py --impl reference --gpus N --steps K --warmup W   # the reference's math on the host CPU cores
+    python bench.py ... --dump-outputs DIR    # also write the last timed step's outputs as DIR/<name>.npy (float32)
 
 One "step" = one complete pass of the hot path over one synthetic 16-frame clip: CLIP embed + VAE encode of the
 reference image, ReferenceNet write pass, PoseGuider, 25 CFG DDIM steps of the denoising UNet (reference attention +
@@ -26,6 +27,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the source tree as it found it (it may be read-only)
 
 METRIC = "denoised frames/sec @512x512 L=16 steps=25"
 W = H = 512
@@ -449,10 +451,12 @@ def run_product(args):
     barrier()
     e0.record()
     for _ in range(args.steps):
-        device_step()
+        video = device_step()
     e1.record()
     barrier()
     ms_step = e0.elapsed_time(e1) / args.steps
+    # what the caller of the timed path receives from its last step: the decoded video and the final latents
+    outputs = {"video": video.float().cpu(), "latents": pipe.last_latents.float().cpu()} if args.dump_outputs else None
     launches = (ops.KERNEL_LAUNCHES - n0)
     phases = pipe.collect_timings()
     clocks = sampler.stop() if rank == 0 else {}
@@ -555,8 +559,25 @@ def run_product(args):
         if args.cpu_baseline and world == 1:
             line["cpu_baseline"] = cpu_baseline_sample(args.cpu_threads)
         print(json.dumps(line))
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
     if world > 1:
         torch.distributed.destroy_process_group()
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(directory, outputs):
+    """Writes each output as <directory>/<name>.npy in float32, so that two builds can be compared output for output on
+    the same (seeded, run-to-run identical) inputs."""
+    import numpy as np
+    total = sum(t.numel() * 4 for t in outputs.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError(f"outputs take {total} bytes, more than the {DUMP_LIMIT_BYTES} bytes --dump-outputs writes")
+    os.makedirs(directory, exist_ok=True)
+    for name, t in outputs.items():
+        np.save(os.path.join(directory, name + ".npy"), t.numpy().astype(np.float32))
 
 
 # ----------------------------------------------------------------------------------------------------------------
@@ -639,15 +660,11 @@ def run_reference(args):
     """--impl reference: the reference's own CPU implementation of the path. The reference is pure PyTorch + diffusers;
     diffusers is not installable offline and /root/reference does not travel to the GPU box, so the arm times
     oracle/functional.py (the restatement pinned against the unmodified reference wiring) on the host cores, at the real
-    geometry (see cpu_baseline_sample). Rank 0 only; one sample per `step` (at most 2: a sample is minutes of CPU time)."""
+    geometry (see cpu_baseline_sample). Rank 0 only; one sample per `step` (a sample is minutes of CPU time)."""
     if int(os.environ.get("RANK", "0")) != 0:
         return
     threads = args.cpu_threads or min(os.cpu_count() or 1, 32)
-    vals = []
-    for _ in range(max(1, min(args.steps, 2))):
-        vals.append(cpu_baseline_sample(threads))
-        if sum(v["seconds"]["ddim_step_L4"] for v in vals) > 60:
-            break
+    vals = [cpu_baseline_sample(threads) for _ in range(args.steps)]
     best = max(vals, key=lambda d: d["value"])
     v = best["value"]
     line = {"impl": "reference", "metric": METRIC, "value": v, "unit": "frames/s", "n_gpus": args.gpus,
@@ -671,7 +688,15 @@ def main():
     ap.add_argument("--no-c4", dest="c4", action="store_false", help="skip the 128-frame strong-scaling leg")
     ap.add_argument("--no-c1", dest="c1", action="store_false", help="skip the C1 (L=4, 10 steps) like-for-like leg")
     ap.add_argument("--cpu-threads", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's video and latents as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.warmup < 0:
+        ap.error("--warmup must not be negative")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the product arm's outputs; the reference arm returns timings only")
     if args.impl == "reference":
         run_reference(args)
     else:

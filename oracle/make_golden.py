@@ -42,8 +42,9 @@ def _load(model, seed):
     return sd
 
 
-def case_unet3d(name, chans, Fr, h, w, timestep, seeds=(101, 102, 103)):
-    """ReferenceNet write pass + denoising UNet read pass under CFG, as pipeline_pose2vid_long.py:475-544 wires them."""
+def case_unet3d(name, chans, Fr, h, w, timestep, seeds=(101, 102, 103), stride=1):
+    """ReferenceNet write pass + denoising UNet read pass under CFG, as pipeline_pose2vid_long.py:475-544 wires them.
+    Stores every `stride`-th latent row and column of the output (fixtures stay under 1 MB)."""
     ref_import.activate()
     from src.models.mutual_self_attention import ReferenceAttentionControl
     t0 = time.time()
@@ -63,7 +64,8 @@ def case_unet3d(name, chans, Fr, h, w, timestep, seeds=(101, 102, 103)):
         out = unet3d(sample, torch.tensor(timestep), encoder_hidden_states=ehs, pose_cond_fea=pose,
                      return_dict=False)[0]
     torch.save(dict(case=name, chans=tuple(chans), frames=Fr, h=h, w=w, timestep=timestep, seeds=tuple(seeds),
-                    out=out.float().contiguous(), torch_version=str(torch.__version__),
+                    out=out[..., ::stride, ::stride].float().contiguous(), out_shape=tuple(out.shape), out_stride=stride,
+                    torch_version=str(torch.__version__),
                     generator="reference src/models via oracle/diffusers_shim, fp32 CPU"),
                os.path.join(GOLDEN, name + ".pt"))
     print(f"{name}: out {tuple(out.shape)} |out|={out.norm():.4f} in {time.time() - t0:.1f}s")
@@ -201,7 +203,8 @@ def case_pipeline_c1(name="pipeline_c1_full", P=PIPE_C1_FULL):
     wall = time.perf_counter() - t1
     videos = out.videos
     torch.save(dict(case=name, params={k: v for k, v in P.items()}, final_latents=lat_trace[-1].float(),
-                    first_step_latents=lat_trace[0].float(), video_frames=videos[:, :, [0, P["L"] - 1]].half(),
+                    first_step_latents=lat_trace[0].float(), video_stride=4,      # every 4th pixel row and column
+                    video_frames=videos[:, :, [0, P["L"] - 1], ::4, ::4].half(),
                     video_frame_means=videos.mean(dim=(0, 1, 3, 4)).float(), torch_version=str(torch.__version__),
                     cpu_reference=dict(wall_s=wall, frames=P["L"], frames_per_s=P["L"] / wall,
                                        threads=torch.get_num_threads(), nproc=os.cpu_count(),
@@ -215,12 +218,151 @@ def case_pipeline_c1(name="pipeline_c1_full", P=PIPE_C1_FULL):
           f"phases={ {k: round(v, 1) for k, v in timer.seconds.items()} } total {time.time() - t0:.1f}s")
 
 
+UNIT_CHANS = (64, 128, 256, 256)
+
+
+def unit_unet_inputs():
+    """Inputs of the plain denoising-UNet check of tests/test_oracle_vs_reference.py (no reference attention)."""
+    g = torch.Generator().manual_seed(3)
+    x = torch.randn(2, 4, 3, 16, 16, generator=g)
+    ehs = torch.randn(2, 1, 768, generator=g)
+    pose = [torch.randn(2, c, 3, s, s, generator=g) for c, s in [(64, 16), (64, 8), (128, 4), (256, 2), (256, 2)]]
+    return x, ehs, pose
+
+
+def unit_ref_attention_inputs():
+    """Inputs of the ReferenceNet write / denoising-UNet read check under CFG; 16 frames per branch because the reference
+    hard-codes a 16-frame uc_mask (mutual_self_attention.py:77-85)."""
+    g = torch.Generator().manual_seed(4)
+    x = torch.randn(1, 4, 16, 8, 8, generator=g).repeat(2, 1, 1, 1, 1)
+    clip = torch.randn(1, 768, generator=g)
+    ehs = torch.cat([torch.zeros_like(clip), clip], 0).unsqueeze(1)
+    ref_lat = torch.randn(1, 4, 8, 8, generator=g)
+    return x, ehs, ref_lat
+
+
+def unit_pose_guider_inputs():
+    """Pose maps of the PoseGuider check, and the reference-pose image the reference's forward takes (and ignores)."""
+    g = torch.Generator().manual_seed(6)
+    return torch.randn(2, 3, 2, 128, 128, generator=g), torch.randn(1, 3, 128, 128, generator=g)
+
+
+# context_overlap == context_size * hop (zero range step) and larger (negative step) in the last two
+UNIFORM_ARGS = [(0, 25, n, 16, 1, 4) for n in (4, 16, 24, 128)] + \
+    [(0, 25, 24, 16, 2, 4), (3, 25, 50, 16, 3, 4), (0, 25, 40, 16, 1, 16), (0, 25, 40, 16, 1, 20)]
+FILM_CASES = [(1, 5), (2, 3)]             # (batch, frames) of the frame-interpolation check, 1..5 inserted frames each
+POSE_CASES = [(0, 64, 37, True), (1, 128, 61, False)]      # (seed, latent_dim, frames, only_last_features)
+
+
+def pose_model_weights(model, seed):
+    """Seeded weights of everything but the audio encoder of an Audio2PoseModel; fan-in scaled so that the 8 decoder layers
+    move the result (the default init is close to the identity)."""
+    sd = {k: v for k, v in model.state_dict().items() if not k.startswith("audio_encoder.")}
+    return randomize_state_dict(sd, seed=seed, std=1.0)
+
+
+def _uniform_outcome(uniform, args):
+    try:
+        return [list(map(int, w)) for w in uniform(*args)]
+    except ValueError:
+        return "ValueError"
+
+
+def case_reference_units(name="reference_units"):
+    """Outputs of the UNMODIFIED reference's modules and helpers at unit-test sizes, for the checks that compare the CPU
+    oracle or a host-side rewrite with the reference: denoising UNet (plain and with reference attention), PoseGuider,
+    the context-window scheduler, the FILM frame-interpolation loop (on the tests' stand-in network) and the head-pose
+    decoder (Audio2PoseModel.infer). Also the constructor / call / state-dict surface of the reference classes."""
+    import gzip
+    import importlib.util
+    import json
+    import tempfile
+    ref_import.activate()
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    from src.models.mutual_self_attention import ReferenceAttentionControl
+    from src.pipelines.context import uniform
+    from test_dropin_conformance import _probe
+    from test_host_cpu import _StandInFilm
+    t0 = time.time()
+    G = dict(case=name, torch_version=str(torch.__version__), generator="reference src/ via oracle/diffusers_shim, fp32 CPU")
+    torch.manual_seed(0)
+    unet3d, unet2d = ref_import.build_unet3d(UNIT_CHANS), ref_import.build_unet2d(UNIT_CHANS)
+    _load(unet3d, 1)
+    _load(unet2d, 2)
+    x, ehs, pose = unit_unet_inputs()
+    with torch.no_grad():
+        G["unet3d_plain"] = unet3d(x, torch.tensor(500), encoder_hidden_states=ehs, pose_cond_fea=pose,
+                                   return_dict=False)[0]
+    x, ehs, ref_lat = unit_ref_attention_inputs()
+    writer = ReferenceAttentionControl(unet2d, do_classifier_free_guidance=True, mode="write", batch_size=1,
+                                       fusion_blocks="full")
+    reader = ReferenceAttentionControl(unet3d, do_classifier_free_guidance=True, mode="read", batch_size=1,
+                                       fusion_blocks="full")
+    with torch.no_grad():
+        unet2d(ref_lat.repeat(2, 1, 1, 1), torch.zeros((), dtype=torch.long), encoder_hidden_states=ehs, return_dict=False)
+        reader.update(writer, dtype=torch.float32)
+        G["unet3d_ref_attention"] = unet3d(x, torch.tensor(959), encoder_hidden_states=ehs, return_dict=False)[0]
+    pg = ref_import.build_pose_guider(64)
+    _load(pg, 5)
+    pg.train()  # the scripts never call .eval(): BatchNorm uses batch statistics
+    with torch.no_grad():    # every second row and column of each output: the stored sample stays small
+        G["pose_guider"] = [t[..., ::2, ::2].clone() for t in pg(*unit_pose_guider_inputs())]
+    G["uniform"] = [(args, _uniform_outcome(uniform, args)) for args in UNIFORM_ARGS]
+
+    spec = importlib.util.spec_from_file_location(
+        "_ref_frame_interpolation", os.path.join(ref_import.REFERENCE_ROOT, "src", "utils", "frame_interpolation.py"))
+    film = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(film)
+    cuda = torch.Tensor.cuda
+    torch.Tensor.cuda = lambda self, *a, **k: self      # the reference hard-codes .cuda()
+    try:
+        g = torch.Generator().manual_seed(3)
+        G["film"] = []
+        for bs, frames in FILM_CASES:
+            video = torch.rand((bs, 3, frames, 8, 12), generator=g)              # fp32, not fp16-representable
+            G["film"].append(dict(video=video, out=[film.batch_images_interpolation_tool(video, _StandInFilm(), n)
+                                                    for n in range(1, 6)]))
+    finally:
+        torch.Tensor.cuda = cuda
+
+    from transformers import Wav2Vec2Config
+    from src.audio_models.pose_model import Audio2PoseModel
+    G["pose_infer"] = []
+    with tempfile.TemporaryDirectory() as cfg_dir:
+        cfg = Wav2Vec2Config(hidden_size=64, num_hidden_layers=2, num_attention_heads=4, intermediate_size=128,
+                             conv_dim=(32, 32, 32), conv_stride=(5, 4, 2), conv_kernel=(10, 4, 2),
+                             num_feat_extract_layers=3, num_conv_pos_embeddings=16, num_conv_pos_embedding_groups=4)
+        cfg._attn_implementation = "eager"        # the reference's wav2vec2 wrapper asks for attention maps
+        cfg.save_pretrained(cfg_dir)
+        for seed, latent, T, only_last in POSE_CASES:
+            torch.manual_seed(seed)
+            m = Audio2PoseModel(dict(latent_dim=latent, model_path=cfg_dir, only_last_fetures=only_last,
+                                     from_pretrained=False, out_dim=6)).eval()
+            m.audio_encoder.config._attn_implementation = "eager"
+            m.load_state_dict(pose_model_weights(m, seed), strict=False)
+            with torch.no_grad():
+                audio = torch.randn(1, 16000)
+                emb = m.audio_encoder(audio, seq_len=T, output_hidden_states=True)
+                want = m.infer(audio, T, id_seed=torch.tensor([7]))
+            spread = (want[0, 1:] - want[0, :-1]).abs().mean().item()
+            assert spread > 1e-3, "degenerate reference output: the check would prove nothing"
+            features = emb.last_hidden_state if only_last else torch.stack(emb.hidden_states)
+            G["pose_infer"].append(dict(seed=seed, latent=latent, frames=T, only_last=only_last, features=features,
+                                        pe=m.PPE.pe[:, :T].clone(), out=want))
+            G["pose_biased_mask"] = m.biased_mask[:, :T, :T].clone()     # the same buffer in every model; largest T last
+    torch.save(G, os.path.join(GOLDEN, name + ".pt"))
+    with gzip.open(os.path.join(GOLDEN, "dropin_reference_surface.json.gz"), "wt") as f:
+        json.dump(_probe("reference"), f, sort_keys=True)
+    print(f"{name}: written in {time.time() - t0:.1f}s")
+
+
 CASES = {
+    "reference_units": case_reference_units,
     "pipeline_small": case_pipeline,
     "pipeline_c1_full": case_pipeline_c1,
     # the benchmarked geometry (BASELINE.json configs[1]): full width, 64x64 latents, one 16-frame window under CFG
     "unet3d_full_f16_64x64": lambda: case_unet3d("unet3d_full_f16_64x64", (320, 640, 1280, 1280), 16, 64, 64, 479,
-                                                  seeds=(121, 122, 123)),
+                                                  seeds=(121, 122, 123), stride=2),
     # full SD1.5 width (the real model size), 256x256-pixel equivalent latents, 4-frame window
     "unet3d_full_f4_32x32": lambda: case_unet3d("unet3d_full_f4_32x32", (320, 640, 1280, 1280), 4, 32, 32, 479),
     # reduced width, 16-frame window (temporal attention at the production window length), non-square latent

@@ -12,12 +12,18 @@ def available():
     return os.path.isdir(os.path.join(REFERENCE_ROOT, "src", "models"))
 
 
+def activate_shim():
+    """Only the diffusers shim (part of this repository): what the checks that need no reference module import."""
+    if SHIM not in sys.path:
+        sys.path.insert(0, SHIM)
+
+
 def activate():
     if not available():
         raise RuntimeError(f"reference not found at {REFERENCE_ROOT}")
-    for p in (SHIM, REFERENCE_ROOT):
-        if p not in sys.path:
-            sys.path.insert(0, p)
+    activate_shim()
+    if REFERENCE_ROOT not in sys.path:
+        sys.path.insert(0, REFERENCE_ROOT)
 
 
 MOTION_KWARGS = dict(num_attention_heads=8, num_transformer_block=1,

@@ -1,17 +1,16 @@
 """The drop-in boundary (SURVEY.md 8b): `dropin/src/...` must expose, under the reference's import paths, classes whose
 constructor / forward / __call__ signatures accept everything the reference's scripts pass, and whose state-dict keys are
 exactly the reference's (so denoising_unet.pth / motion_module.pth / reference_unet.pth / pose_guider.pth load). Compared
-against the UNMODIFIED reference classes imported through oracle/diffusers_shim; needs /root/reference (authoring
-container; skipped on the GPU box). Each side is imported in its own interpreter: both define a top-level `src` package."""
+against the surface of the UNMODIFIED reference classes (imported through oracle/diffusers_shim), stored in
+tests/golden/dropin_reference_surface.json.gz by oracle/make_golden.py. The probe runs in its own interpreter: the drop-in
+and the reference both define a top-level `src` package."""
+import gzip
 import json
 import os
 import subprocess
 import sys
 
-import pytest
-
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REFERENCE = os.environ.get("ANIPORTRAIT_REFERENCE", "/root/reference")
 
 PROBE = r'''
 import inspect, json, sys
@@ -82,16 +81,19 @@ print("PROBE_JSON" + json.dumps(res))
 
 
 def _probe(side):
+    """side "product": the drop-in classes; side "reference": the reference's (oracle/make_golden.py stores that result)."""
+    from oracle import ref_import
     r = subprocess.run([sys.executable, "-c", PROBE, side, ROOT], capture_output=True, text=True, timeout=600,
-                       cwd=ROOT if side == "product" else REFERENCE)
+                       cwd=ROOT if side == "product" else ref_import.REFERENCE_ROOT)
     assert r.returncode == 0, r.stderr[-3000:]
     line = [ln for ln in r.stdout.splitlines() if ln.startswith("PROBE_JSON")][-1]
     return json.loads(line[len("PROBE_JSON"):])
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REFERENCE, "src", "models")), reason="reference tree not present")
 def test_dropin_surface_matches_reference_classes():
-    ref, ours = _probe("reference"), _probe("product")
+    with gzip.open(os.path.join(ROOT, "tests", "golden", "dropin_reference_surface.json.gz"), "rt") as f:
+        ref = json.load(f)
+    ours = _probe("product")
     # 1. every parameter the reference accepts exists on ours, in the same position, with the same default
     for name, rsig in ref["sig"].items():
         osig = ours["sig"][name]

@@ -2,8 +2,8 @@
 window scheduler, image pre-processing, weight repacking, state-dict surface) against the oracle; world_size-2 gloo test
 of the window-sharded denoising step."""
 import os
-import subprocess
 import sys
+import types
 
 import numpy as np
 import pytest
@@ -18,6 +18,11 @@ from oracle import functional as OF  # noqa: E402
 def rel_l2(a, b):
     a, b = a.detach().float(), b.detach().float()
     return ((a - b).norm() / (b.norm() + 1e-12)).item()
+
+
+def _reference_units():
+    """Outputs of the unmodified reference at unit-test sizes (oracle/make_golden.py reference_units)."""
+    return torch.load(os.path.join(ROOT, "tests", "golden", "reference_units.pt"))
 
 
 def test_library_exports_every_declared_symbol():
@@ -252,14 +257,12 @@ def test_window_scheduler_degenerate_overlap_fails_like_the_reference():
     with pytest.raises(ValueError):
         list(uniform(0, 25, 40, 16, 1, 16))
     assert list(uniform(0, 25, 40, 16, 1, 20)) == []
-    if os.path.isdir("/root/reference/src/pipelines"):
-        sys.path.insert(0, "/root/reference")
-        from src.pipelines.context import uniform as ref_uniform
-        with pytest.raises(ValueError):
-            list(ref_uniform(0, 25, 40, 16, 1, 16))
-        assert list(ref_uniform(0, 25, 40, 16, 1, 20)) == []
-        for args in [(0, 25, 24, 16, 2, 4), (3, 25, 50, 16, 3, 4), (0, 25, 128, 16, 1, 4)]:
-            assert list(uniform(*args)) == [list(map(int, w)) for w in ref_uniform(*args)]
+    # what the reference's uniform() returned (or raised) for the same arguments
+    ref = dict(_reference_units()["uniform"])
+    assert ref[(0, 25, 40, 16, 1, 16)] == "ValueError"
+    assert ref[(0, 25, 40, 16, 1, 20)] == []
+    for args in [(0, 25, 24, 16, 2, 4), (3, 25, 50, 16, 3, 4), (0, 25, 128, 16, 1, 4)]:
+        assert list(uniform(*args)) == ref[args]
 
 
 def test_repeated_frame_in_a_window_counts_once():
@@ -514,19 +517,14 @@ class _StandInFilm(torch.nn.Module):
         return mix + 0.3 * torch.sin(7 * torch.roll(x0, 1, -1) - 5 * torch.roll(x1, 1, -2) + 3 * t) - 0.05
 
 
-def test_frame_interpolation_matches_reference_order_and_values(monkeypatch):
+def test_frame_interpolation_matches_reference_order_and_values():
     """N2 (SURVEY.md 8f): the batched `-acc` wrapper returns the frames of the unmodified reference
     src/utils/frame_interpolation.py:23-69 (one network call per inserted frame and pair, host round trips) — same insertion
-    order, same dt bit patterns, same clamping, same pass-through of the given frames — with `inter_frames` network calls."""
-    import importlib.util
-    ref_path = "/root/reference/src/utils/frame_interpolation.py"
-    if not os.path.exists(ref_path):
-        pytest.skip("reference checkout not present (authoring container only)")
-    spec = importlib.util.spec_from_file_location("_ref_frame_interpolation", ref_path)
-    ref = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref)
-    monkeypatch.setattr(torch.Tensor, "cuda", lambda self, *a, **k: self)     # the reference hard-codes .cuda()
+    order, same dt bit patterns, same clamping, same pass-through of the given frames — with `inter_frames` network calls.
+    The reference's frames on this stand-in network are stored in tests/golden/reference_units.pt."""
     from aniportrait_b200.pipelines.frame_interpolation import batch_images_interpolation_tool, insertion_schedule
+    gold = _reference_units()["film"]
+    assert len(gold) == 2
 
     class Counting(_StandInFilm):
         calls = 0
@@ -536,11 +534,11 @@ def test_frame_interpolation_matches_reference_order_and_values(monkeypatch):
             assert x0.dtype == torch.float16 and dt.dtype == torch.float16
             return super().forward(x0, x1, dt)
 
-    g = torch.Generator().manual_seed(3)
-    for bs, frames in [(1, 5), (2, 3)]:
-        video = torch.rand((bs, 3, frames, 8, 12), generator=g)              # fp32, not fp16-representable
+    for (bs, frames), case in zip([(1, 5), (2, 3)], gold):
+        video = case["video"]                                                 # fp32, not fp16-representable
+        assert video.shape == (bs, 3, frames, 8, 12)
         for n in range(1, 6):
-            want = ref.batch_images_interpolation_tool(video, _StandInFilm(), inter_frames=n)
+            want = case["out"][n - 1]
             Counting.calls = 0
             got = batch_images_interpolation_tool(video, Counting(), inter_frames=n)
             assert Counting.calls == n                                        # (frames - 1) * n in the reference
@@ -553,48 +551,55 @@ def test_frame_interpolation_matches_reference_order_and_values(monkeypatch):
     assert torch.equal(batch_images_interpolation_tool(video, _StandInFilm(), 0), video)
 
 
-def test_kv_cached_pose_infer_matches_reference_infer(tmp_path):
+class _PoseModelStandIn(torch.nn.Module):
+    """The attributes of the reference's Audio2PoseModel (src/audio_models/pose_model.py:56-89) that infer reads, made of
+    torch modules with the reference's hyper-parameters (8 post-norm decoder layers, 8 heads, feed-forward 2 * latent,
+    batch_first); its audio encoder returns the features the reference's wav2vec2 produced for the stored case."""
+
+    def __init__(self, case, biased_mask):
+        super().__init__()
+        E, feats = case["latent"], case["features"]
+        self.out_dim = 6
+        self._only_last_features = case["only_last"]
+        self.pose_map = torch.nn.Linear(6, E)
+        self.in_fn = torch.nn.Linear(feats.shape[-1], E)
+        self.PPE = torch.nn.Module()
+        self.PPE.register_buffer("pe", case["pe"])
+        self.biased_mask = biased_mask
+        layer = torch.nn.TransformerDecoderLayer(d_model=E, nhead=8, dim_feedforward=2 * E, batch_first=True)
+        self.transformer_decoder = torch.nn.TransformerDecoder(layer, num_layers=8)
+        self.pose_map_r = torch.nn.Linear(E, 6)
+        self.id_embed = torch.nn.Embedding(100, E)
+        if case["only_last"]:
+            enc = types.SimpleNamespace(last_hidden_state=feats, hidden_states=None)
+        else:
+            enc = types.SimpleNamespace(last_hidden_state=feats[-1], hidden_states=tuple(feats))
+        self.audio_encoder = lambda input_value, seq_len, output_hidden_states: enc
+
+
+def test_kv_cached_pose_infer_matches_reference_infer():
     """N3 (SURVEY.md 8f): the incremental (KV-cached, one-key cross-attention precomputed) head-pose decoder returns what the
     UNMODIFIED reference Audio2PoseModel.infer (src/audio_models/pose_model.py:97-124) computes by re-decoding all tokens at
-    every frame — same module instance, seeded random weights, CPU fp32."""
-    if not os.path.isdir("/root/reference/src/audio_models"):
-        pytest.skip("reference checkout not present (authoring container only)")
-    script = r'''
-import sys, torch
-sys.path.insert(0, "/root/reference"); sys.path.insert(0, sys.argv[2])
-from transformers import Wav2Vec2Config
-cfg = Wav2Vec2Config(hidden_size=64, num_hidden_layers=2, num_attention_heads=4, intermediate_size=128,
-                     conv_dim=(32, 32, 32), conv_stride=(5, 4, 2), conv_kernel=(10, 4, 2), num_feat_extract_layers=3,
-                     num_conv_pos_embeddings=16, num_conv_pos_embedding_groups=4)
-cfg._attn_implementation = "eager"        # the reference's wav2vec2 wrapper asks for attention maps
-cfg.save_pretrained(sys.argv[1])
-from src.audio_models.pose_model import Audio2PoseModel
-from aniportrait_b200.audio_models import enable_kv_cache, kv_cached_infer
-worst = 0.0
-for seed, latent, T, only_last in [(0, 64, 37, True), (1, 128, 61, False)]:
-    torch.manual_seed(seed)
-    m = Audio2PoseModel(dict(latent_dim=latent, model_path=sys.argv[1], only_last_fetures=only_last,
-                             from_pretrained=False, out_dim=6)).eval()
-    m.audio_encoder.config._attn_implementation = "eager"
-    with torch.no_grad():
-        for p in m.transformer_decoder.parameters():          # default init is near-identity: make the layers matter
-            if p.dim() > 1:
-                p.mul_(3.0)
-        audio = torch.randn(1, 16000)
-        want = m.infer(audio, T, id_seed=torch.tensor([7]))
-        got = kv_cached_infer(m, audio, T, id_seed=torch.tensor([7]))
-        enable_kv_cache(m)
-        again = m.infer(audio, T, id_seed=torch.tensor([7]))
-    assert got.shape == want.shape == (1, T, 6), (got.shape, want.shape)
-    assert torch.equal(got, again)
-    err = ((got - want).norm() / want.norm()).item()
-    spread = (want[0, 1:] - want[0, :-1]).abs().mean().item()
-    assert spread > 1e-3, "degenerate reference output: the test would prove nothing"
-    worst = max(worst, err)
-print("RESULT", worst)
-'''
-    r = subprocess.run([sys.executable, "-c", script, str(tmp_path), ROOT], capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0, r.stderr[-3000:]
-    worst = float([ln for ln in r.stdout.splitlines() if ln.startswith("RESULT")][-1].split()[1])
+    every frame — seeded weights, CPU fp32. The reference's result, audio features and mask / positional-encoding buffers
+    are stored in tests/golden/reference_units.pt."""
+    from oracle.make_golden import POSE_CASES, pose_model_weights
+    from aniportrait_b200.audio_models import enable_kv_cache, kv_cached_infer
+    gold = _reference_units()
+    assert len(gold["pose_infer"]) == len(POSE_CASES)
+    worst = 0.0
+    for case in gold["pose_infer"]:
+        T = case["frames"]
+        m = _PoseModelStandIn(case, gold["pose_biased_mask"][:, :T, :T]).eval()
+        m.load_state_dict(pose_model_weights(m, case["seed"]))
+        want = case["out"]
+        with torch.no_grad():
+            got = kv_cached_infer(m, None, T, id_seed=torch.tensor([7]))
+            enable_kv_cache(m)
+            again = m.infer(None, T, id_seed=torch.tensor([7]))
+        assert got.shape == want.shape == (1, T, 6), (got.shape, want.shape)
+        assert torch.equal(got, again)
+        spread = (want[0, 1:] - want[0, :-1]).abs().mean().item()
+        assert spread > 1e-3, "degenerate reference output: the test would prove nothing"
+        worst = max(worst, ((got - want).norm() / want.norm()).item())
     print(f"kv-cached pose decoder vs reference re-decoding: rel-L2 {worst:.2e}")
     assert worst < 1e-4
