@@ -33,7 +33,7 @@
 namespace ap {
 
 enum { A_GEMM = 0, A_CONV_S1 = 1, A_CONV_S2 = 2 };
-enum { EPI_LINEAR = 0, EPI_GEGLU = 1 };
+enum { EPI_LINEAR = 0, EPI_GEGLU = 1, EPI_GELU = 2 };   // EPI_GELU: out = gelu_erf(acc + bias), no residual / statistics
 
 struct GemmParams {
   int M, N;                // output rows; weight rows (N % BN == 0)
@@ -469,6 +469,10 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA1, const __grid_constant__ CU
                 v[4 * j + 0] += b.x; v[4 * j + 1] += b.y; v[4 * j + 2] += b.z; v[4 * j + 3] += b.w;
               }
             }
+            if (EPI == EPI_GELU) {
+#pragma unroll
+              for (int j = 0; j < 32; ++j) v[j] = gelu_erf(v[j]);
+            }
             if (has_res) {
               mbar_wait(rbar, rphase);
               rphase ^= 1;
@@ -608,6 +612,10 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA1, const __grid_constant__ CU
             v[4 * j + 0] += b.x; v[4 * j + 1] += b.y; v[4 * j + 2] += b.z; v[4 * j + 3] += b.w;
           }
         }
+        if (EPI == EPI_GELU) {
+#pragma unroll
+          for (int j = 0; j < 32; ++j) v[j] = gelu_erf(v[j]);
+        }
         if (EPI == EPI_GEGLU) {
           // interleaved weights: columns [0,16) = value half, [16,32) = gate half of the same 16 outputs
           const int ocol = ncol >> 1;
@@ -718,6 +726,7 @@ static int launch_gemm(const CUtensorMap& a1, const CUtensorMap& a2, const CUten
 
 // Tile-width choice: wider tiles re-use the A operand more (less L2 traffic per FLOP) but give fewer tiles; small-M
 // problems (16x16 / 8x8 levels) prefer narrower tiles to fill the 148 SMs and reduce wave-quantisation loss.
+// geglu (also used for GELU): only tiles that are multiples of 64 columns
 static int pick_bn(int N, int forced, long long m_tiles, bool geglu = false) {
   if (forced > 0) return forced;
   const int cand[5] = {256, 160, 128, 64, 32};
@@ -765,6 +774,17 @@ static int dispatch(int bn, int epi, int cg, const CUtensorMap& a1, const CUtens
   case BN_:                                                                              \
     return epi == EPI_GEGLU ? launch_gemm<BN_, EPI_GEGLU, 2>(a1, a2, b, to, tr, p, stream) \
                             : launch_gemm<BN_, EPI_LINEAR, 2>(a1, a2, b, to, tr, p, stream);
+  if (epi == EPI_GELU) {   // tiles that are multiples of 64 columns only (pick_bn never offers 160 / 32 for GELU)
+    if (cg == 2) {
+      if (bn == 256) return launch_gemm<256, EPI_GELU, 2>(a1, a2, b, to, tr, p, stream);
+      if (bn == 128) return launch_gemm<128, EPI_GELU, 2>(a1, a2, b, to, tr, p, stream);
+      return fail(AP_ERR_INVALID, "gemm: unsupported 2-CTA BLOCK_N %d with GELU", bn);
+    }
+    if (bn == 256) return launch_gemm<256, EPI_GELU, 1>(a1, a2, b, to, tr, p, stream);
+    if (bn == 128) return launch_gemm<128, EPI_GELU, 1>(a1, a2, b, to, tr, p, stream);
+    if (bn == 64) return launch_gemm<64, EPI_GELU, 1>(a1, a2, b, to, tr, p, stream);
+    return fail(AP_ERR_INVALID, "gemm: unsupported BLOCK_N %d with GELU (multiples of 64 only)", bn);
+  }
   if (cg == 2) {
     switch (bn) {
       AP_CASE2(256)
@@ -845,8 +865,8 @@ static int apply_ext(GemmParams& p, const ap_epilogue_ext* ext, int epi, long lo
 using namespace ap;
 
 extern "C" int ap_gemm_row_stat_parts(long long M, int N, int K, int flags, int block_n) {
-  const int epi = (flags & AP_GEMM_GEGLU) ? EPI_GEGLU : EPI_LINEAR;
-  const int bn = pick_bn(N, block_n, (M + 127) / 128, epi == EPI_GEGLU);
+  const int epi = (flags & AP_GEMM_GEGLU) ? EPI_GEGLU : ((flags & AP_GEMM_GELU) ? EPI_GELU : EPI_LINEAR);
+  const int bn = pick_bn(N, block_n, (M + 127) / 128, epi != EPI_LINEAR);
   if (bn <= 0 || N % bn != 0) return fail(AP_ERR_INVALID, "gemm: N=%d not tileable (block_n=%d)", N, block_n);
   GemmParams p{};
   p.num_m_tiles = (int)((M + 127) / 128);
@@ -865,9 +885,11 @@ extern "C" int ap_gemm_f16(const void* a, long long lda, int K1, const void* a2,
   AP_REQUIRE(M > 0 && N > 0 && K1 > 0, "gemm: bad shape M=%lld N=%d K1=%d", M, N, K1);
   AP_REQUIRE(K1 % 64 == 0 || (a2 == nullptr), "gemm: K1 must be a multiple of 64 when a second source follows");
   AP_REQUIRE((lda % 8) == 0 && (a2 == nullptr || (lda2 % 8) == 0), "gemm: lda must be a multiple of 8 elements");
-  const int epi = (flags & AP_GEMM_GEGLU) ? EPI_GEGLU : EPI_LINEAR;
-  const int bn = pick_bn(N, block_n, (M + 127) / 128, epi == EPI_GEGLU);
-  AP_REQUIRE(epi != EPI_GEGLU || (bn > 0 && bn % 64 == 0), "gemm: GEGLU needs a BLOCK_N multiple of 64");
+  AP_REQUIRE(!((flags & AP_GEMM_GEGLU) && (flags & AP_GEMM_GELU)), "gemm: AP_GEMM_GEGLU and AP_GEMM_GELU exclude each other");
+  const int epi = (flags & AP_GEMM_GEGLU) ? EPI_GEGLU : ((flags & AP_GEMM_GELU) ? EPI_GELU : EPI_LINEAR);
+  AP_REQUIRE(epi != EPI_GELU || residual == nullptr, "gemm: no residual with the GELU epilogue");
+  const int bn = pick_bn(N, block_n, (M + 127) / 128, epi != EPI_LINEAR);
+  AP_REQUIRE(epi == EPI_LINEAR || (bn > 0 && bn % 64 == 0), "gemm: GEGLU / GELU need a BLOCK_N multiple of 64");
   AP_REQUIRE(bn > 0 && N % bn == 0, "gemm: N=%d not tileable (block_n=%d)", N, block_n);
   const long long K = (long long)K1 + (a2 ? K2 : 0);
   AP_REQUIRE((K * 2) % 16 == 0, "gemm: K*2 bytes must be a multiple of 16");

@@ -138,8 +138,9 @@ def _with_stats(out, rs, cs, row_stats, col_stats):
 def gemm(a: torch.Tensor, w: torch.Tensor, bias: torch.Tensor | None = None, residual: torch.Tensor | None = None,
          a2: torch.Tensor | None = None, geglu: bool = False, out: torch.Tensor | None = None,
          bias_group_rows: int = 0, n_valid: int = 0, block_n: int = 0, out_f32: bool = False,
-         row_stats: bool = False, col_stats: bool = False, ln: LNFold | None = None):
+         row_stats: bool = False, col_stats: bool = False, ln: LNFold | None = None, gelu: bool = False):
     """out = [a | a2] @ w.T (+bias) (+residual); a:[M,K1] fp16 (row stride may exceed K1), w:[N,K1+K2] fp16.
+    gelu: out = gelu_erf([a | a2] @ w.T + bias) (no residual).
     row_stats / col_stats: also return the epilogue's RowStats / ColStats of `out` (-> (out, RowStats?, ColStats?)).
     ln: fold a LayerNorm of `a` into this GEMM (see LNFold). bias may be a column slice of a wider fp32 table."""
     _ensure(a)
@@ -166,7 +167,8 @@ def gemm(a: torch.Tensor, w: torch.Tensor, bias: torch.Tensor | None = None, res
         assert bias.is_contiguous() or bias.dim() == 2
     if residual is not None:
         assert residual.dtype == torch.float16 and residual.stride(1) == 1 and residual.shape[0] == M
-    flags = (1 if geglu else 0) | (2 if out_f32 else 0)
+    assert not (gelu and (geglu or residual is not None)), "the GELU epilogue takes no residual and excludes GEGLU"
+    flags = (1 if geglu else 0) | (2 if out_f32 else 0) | (4 if gelu else 0)
     ext, rs, cs = _epilogue_ext(M, N, a.device, row_stats, col_stats, ln, bias, flags, K1 + K2, block_n)
     rc = lib().ap_gemm_f16(ptr(a), LL(a.stride(0)), I(K1), ptr(a2), LL(a2.stride(0) if a2 is not None else 0), I(K2),
                            ptr(w), LL(M), I(N), fptr(bias), LL(bias_group_rows), ptr(residual),
@@ -174,7 +176,8 @@ def gemm(a: torch.Tensor, w: torch.Tensor, bias: torch.Tensor | None = None, res
                            I(nout), I(flags), I(block_n), stream_ptr(), _lib.ext_ptr(ext))
     check(rc, "ap_gemm_f16")
     if SHAPE_LOG is not None:
-        SHAPE_LOG.append(("gemm_geglu" if geglu else "gemm", M, N, K1 + K2, int(residual is not None)))
+        SHAPE_LOG.append(("gemm_geglu" if geglu else ("gemm_gelu" if gelu else "gemm"), M, N, K1 + K2,
+                          int(residual is not None)))
     _count()
     return _with_stats(out, rs, cs, row_stats, col_stats)
 
@@ -589,3 +592,100 @@ def pack_frames_u8(video: torch.Tensor, rescale: bool = False) -> torch.Tensor:
                                   stream_ptr()), "ap_pack_frames_u8")
     _count()
     return out
+
+
+# --------------------------------------------------------------------------------------------------------------
+# audio front-end (wav2vec2 encoder of audio2vid)
+# --------------------------------------------------------------------------------------------------------------
+def wav_conv0_gn_gelu(wav: torch.Tensor, w: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor,
+                      eps: float = 1e-5) -> torch.Tensor:
+    """wav2vec2 feature-extractor layer 0: Conv1d(1, 512, 10, stride 5, no bias) + GroupNorm(512, 512) + GELU.
+    wav: fp32 [S]; w: fp32 [512, 10]; gamma/beta fp32 [512]; returns fp16 channels-last [(S - 10) // 5 + 1, 512]."""
+    _ensure(wav)
+    assert wav.dtype == torch.float32 and wav.dim() == 1 and wav.is_contiguous()
+    assert w.dtype == torch.float32 and w.shape == (512, 10) and w.is_contiguous()
+    assert gamma.dtype == torch.float32 and gamma.numel() == 512 and beta.dtype == torch.float32 and beta.numel() == 512
+    S = wav.numel()
+    if S < 10:
+        raise ValueError(f"wav_conv0_gn_gelu: {S} samples, fewer than the kernel width 10")
+    out = torch.empty((S - 10) // 5 + 1, 512, dtype=torch.float16, device=wav.device)
+    need = lib().ap_wav_conv0_workspace_floats(LL(S))
+    if need < 0:
+        check(need, "ap_wav_conv0_workspace_floats")
+    ws = torch.empty(need, dtype=torch.float32, device=wav.device)
+    check(lib().ap_wav_conv0_gn_gelu_f16(fptr(wav), LL(S), fptr(w), fptr(gamma), fptr(beta), _lib.c_float(eps), fptr(ws),
+                                         LL(ws.numel()), ptr(out), stream_ptr()), "ap_wav_conv0_gn_gelu_f16")
+    _count(3)
+    return out
+
+
+def pack_conv1d_taps(w: torch.Tensor) -> torch.Tensor:
+    """Conv1d weight [Cout, Cin, k] -> [Cout, k * Cin] fp16, tap-major / channel-minor: row o, column t * Cin + c holds
+    w[o, c, t], the order in which a channels-last strided view presents k consecutive input frames."""
+    cout, cin, k = w.shape
+    return w.detach().permute(0, 2, 1).reshape(cout, k * cin).to(torch.float16).contiguous()
+
+
+def conv1d_s2_gelu(x: torch.Tensor, w_packed: torch.Tensor, k: int) -> torch.Tensor:
+    """Conv1d(C, C, k in {2, 3}, stride 2, no bias) + GELU on channels-last x [T_in, C] fp16 as ONE GEMM over strided views of
+    x (no im2col): A row t = frames 2t, 2t+1 (= x viewed as [T_out, 2C] with row stride 2C), plus frame 2t + 2 for k = 3 as the
+    second K source (x from frame 2 on, same row stride). w_packed: pack_conv1d_taps(w). Returns [T_out, C]."""
+    assert k in (2, 3) and x.dtype == torch.float16 and x.is_contiguous() and x.dim() == 2
+    t_in, c = x.shape
+    if t_in < k:
+        raise ValueError(f"conv1d_s2_gelu: {t_in} frames, fewer than the kernel width {k}")
+    t_out = (t_in - k) // 2 + 1
+    # the views end inside x: k = 2 reads frames <= 2 t_out - 1 <= t_in - 1; k = 3 reads frames <= 2 (t_out - 1) + 2 <= t_in - 1
+    a = x.as_strided((t_out, 2 * c), (2 * c, 1))
+    a2 = x.as_strided((t_out, c), (2 * c, 1), x.storage_offset() + 2 * c) if k == 3 else None
+    assert w_packed.shape == (c, k * c)
+    return gemm(a, w_packed, a2=a2, gelu=True)
+
+
+def interp_linear_time(x: torch.Tensor, t_out: int) -> torch.Tensor:
+    """F.interpolate(mode="linear", align_corners=True) along time: x [T_in, C] fp16 -> [t_out, C]."""
+    _ensure(x)
+    assert x.dtype == torch.float16 and x.is_contiguous() and x.dim() == 2 and x.shape[1] % 8 == 0
+    out = torch.empty(int(t_out), x.shape[1], dtype=torch.float16, device=x.device)
+    check(lib().ap_interp_linear_time_f16(ptr(x), I(x.shape[0]), I(x.shape[1]), ptr(out), I(int(t_out)), stream_ptr()),
+          "ap_interp_linear_time_f16")
+    _count()
+    return out
+
+
+POS_CONV_GROUPS, POS_CONV_K = 16, 128
+
+
+def pack_pos_conv_weight(w: torch.Tensor) -> torch.Tensor:
+    """Resolved positional-conv weight [768, 48, 128] (out, in-of-group, tap) -> [16 groups, 128 taps, 48 in, 48 out] fp16."""
+    cout, cin_g, k = w.shape
+    g = POS_CONV_GROUPS
+    assert k == POS_CONV_K and cout == g * cin_g
+    return w.detach().reshape(g, cout // g, cin_g, k).permute(0, 3, 2, 1).to(torch.float16).contiguous()
+
+
+def pos_conv_gelu(x: torch.Tensor, w_packed: torch.Tensor, bias: torch.Tensor) -> torch.Tensor:
+    """x + GELU(grouped positional conv(x) + bias), k = 128, padding 64, last frame dropped. x: [T, 768] fp16."""
+    _ensure(x)
+    assert x.dtype == torch.float16 and x.is_contiguous() and x.dim() == 2 and x.shape[1] == 768
+    assert w_packed.dtype == torch.float16 and w_packed.shape == (16, 128, 48, 48) and w_packed.is_contiguous()
+    assert bias.dtype == torch.float32 and bias.numel() == 768 and bias.is_contiguous()
+    out = torch.empty_like(x)
+    check(lib().ap_pos_conv_gelu_f16(ptr(x), I(x.shape[0]), ptr(w_packed), fptr(bias), ptr(out), stream_ptr()),
+          "ap_pos_conv_gelu_f16")
+    _count()
+    return out
+
+
+def mean_f16(x: torch.Tensor, out_f32: bool = True, out_f16: bool = False):
+    """Mean over the leading dim of fp16 x [n_src, ...], summed in fp32 in order; returns the fp32 and / or fp16 result
+    (a tuple when both are asked for). n_src = 1: an fp16 -> fp32 copy."""
+    _ensure(x)
+    assert x.dtype == torch.float16 and x.is_contiguous() and (out_f32 or out_f16)
+    o32 = torch.empty(x.shape[1:], dtype=torch.float32, device=x.device) if out_f32 else None
+    o16 = torch.empty(x.shape[1:], dtype=torch.float16, device=x.device) if out_f16 else None
+    check(lib().ap_mean_f16(ptr(x), I(x.shape[0]), LL(x[0].numel()), fptr(o32), ptr(o16), stream_ptr()), "ap_mean_f16")
+    _count()
+    if out_f32 and out_f16:
+        return o32, o16
+    return o32 if out_f32 else o16

@@ -30,6 +30,10 @@ extern "C" {
 /* flags for ap_gemm_f16 */
 #define AP_GEMM_GEGLU 1 /* weight rows interleaved [16 value | 16 gate]; out = value * gelu_erf(gate), N/2 columns */
 #define AP_GEMM_OUT_F32 2 /* `out` is fp32 [M, ldo] (used for the small per-step bias tables) */
+/* out = gelu_erf(acc + bias) (bias optional; no residual, no epilogue statistics): the wav2vec2 feature-extractor convolutions
+ * 1-6 (Conv1d without bias + GELUActivation, transformers Wav2Vec2NoLayerNormConvLayer) and each encoder layer's
+ * feed_forward.intermediate_dense + intermediate_act_fn (reference src/audio_models/wav2vec2.py:30,47 -> transformers) */
+#define AP_GEMM_GELU 4
 
 /*
  * Optional epilogue extensions of ap_gemm_f16 / ap_conv3x3_nhwc_f16 (pass NULL for none). They need the TMA epilogue
@@ -214,6 +218,50 @@ int ap_cfg_ddim_step_f16(float* acc, const float* inv_count, int cfg, float guid
  */
 int ap_pack_frames_u8(const void* video, const long long* strides, int B, int F, int H, int W, int rescale, void* out,
                       void* stream);
+
+/*
+ * Audio front-end of audio2vid (reference scripts/audio2vid.py:162,189-195 -> src/audio_models/model.py:58-69,
+ * pose_model.py:97-105 -> wav2vec2.py:13-64): the wav2vec2-base encoder (transformers Wav2Vec2Model with
+ * feat_extract_norm="group") on sm_100a. The transformer layers use ap_gemm_f16 / ap_attention_f16 / ap_layernorm_f16;
+ * the three entry points below are the parts no existing kernel covers. Feature-extractor layers 1-6 (k = 3 / 2,
+ * stride 2, 512 channels, no bias) are ap_gemm_f16 calls with AP_GEMM_GELU over strided views of the channels-last input
+ * (row stride 1024 = two input frames; k = 2: A = x as [T_out, 1024]; k = 3: A = [x as [T_out, 1024] | x from frame 2 on
+ * as [T_out, 512]]) with tap-major weights [512, k * 512]: no im2col buffer, and no TMA box reads past frame T_in - 1.
+ */
+
+/*
+ * Feature-extractor layer 0: Conv1d(1, 512, k = 10, stride 5, no bias) on the raw waveform + GroupNorm(512, 512) (one
+ * channel per group: statistics over time, biased variance) + exact-erf GELU (transformers Wav2Vec2GroupNormConvLayer).
+ * wav: fp32 [S], S >= 10; w: fp32 [512, 10]; gamma/beta: fp32 [512]; out: fp16 [T0, 512] channels-last,
+ * T0 = (S - 10) / 5 + 1. workspace: fp32, at least ap_wav_conv0_workspace_floats(S) floats (per-block partial sums and
+ * the per-channel affine pair): the reduction is atomic-free in a fixed order, double-precision finalize (bit-reproducible).
+ */
+int ap_wav_conv0_workspace_floats(long long S); /* AP_ERR_INVALID if S needs more than 2^31 - 1 floats */
+int ap_wav_conv0_gn_gelu_f16(const float* wav, long long S, const float* w, const float* gamma, const float* beta,
+                             float eps, float* workspace, long long workspace_floats, void* out, void* stream);
+
+/*
+ * F.interpolate(mode="linear", align_corners=True) along time of a channels-last fp16 matrix (reference
+ * src/audio_models/torch_utils.py:17-20, applied at wav2vec2.py:32): x [T_in, C] -> out [T_out, C], C % 8 == 0,
+ * fp32 weights computed as torch does (scale = (T_in - 1) / (T_out - 1), 0 for T_out = 1).
+ */
+int ap_interp_linear_time_f16(const void* x, int T_in, int C, void* out, int T_out, void* stream);
+
+/*
+ * wav2vec2 positional convolution (transformers Wav2Vec2PositionalConvEmbedding + the residual add of Wav2Vec2Encoder):
+ *   out[t] = x[t] + gelu_erf(b + sum_k W_k x[t + k - 64])   on [T, 768], 16 groups of 48 channels, k = 128, padding 64,
+ * the last of the T + 1 conv outputs dropped (Wav2Vec2SamePadLayer). w: the weight-norm-resolved weight packed
+ * [16 groups][128 taps][48 in][48 out] fp16; bias: fp32 [768]. Tensor cores (mma.sync through WMMA), fp32 accumulation,
+ * taps summed in a fixed order. out must not alias x.
+ */
+int ap_pos_conv_gelu_f16(const void* x, int T, const void* w, const float* bias, void* out, void* stream);
+
+/*
+ * out[i] = (sum over s = 0 .. n_src-1 of x[s * n + i]) / n_src, summed in fp32 in order s = 0, 1, ... (the reference's
+ * `sum(hidden_states) / len(hidden_states)`, src/audio_models/model.py:63-66; n_src = 1 is an fp16 -> fp32 copy).
+ * x: fp16 [n_src, n]; out_f32 (fp32 [n]) and/or out_f16 (fp16 [n]) may be NULL.
+ */
+int ap_mean_f16(const void* x, int n_src, long long n, float* out_f32, void* out_f16, void* stream);
 
 #ifdef __cplusplus
 }
