@@ -689,3 +689,73 @@ def mean_f16(x: torch.Tensor, out_f32: bool = True, out_f16: bool = False):
     if out_f32 and out_f16:
         return o32, o16
     return o32 if out_f32 else o16
+
+
+# --------------------------------------------------------------------------------------------------------------
+# face-mesh pose maps (audio2vid / vid2vid conditioning: reference src/utils/pose_util.py, draw_util.py)
+# --------------------------------------------------------------------------------------------------------------
+_F32_F64 = (torch.float32, torch.float64)
+
+
+def _float_operand(t: torch.Tensor, what: str, shape_ok) -> torch.Tensor:
+    _ensure(t)
+    if t.dtype not in _F32_F64 or not shape_ok(t.shape):
+        raise ValueError(f"{what}: expected fp32 / fp64 of the documented shape, got {t.dtype} {tuple(t.shape)}")
+    return t.contiguous()
+
+
+def pose_smooth(x: torch.Tensor, window: int) -> torch.Tensor:
+    """smooth_pose_seq: sliding-window mean over rows of x [L, 6] (fp32 or fp64), bit-identical to numpy's."""
+    x = _float_operand(x, "pose_smooth", lambda s: len(s) == 2 and s[0] > 0 and s[1] == 6)
+    if int(window) < 1:
+        raise ValueError(f"pose_smooth: window {window} < 1")
+    out = torch.empty_like(x)
+    check(lib().ap_pose_smooth(ptr(x), I(x.shape[0]), I(int(window)), I(x.dtype == torch.float64), ptr(out), stream_ptr()),
+          "ap_pose_smooth")
+    _count()
+    return out
+
+
+def project_points(points: torch.Tensor, trans: torch.Tensor, pose: torch.Tensor | None, width: int,
+                   height: int) -> torch.Tensor:
+    """Perspective projection in fp64: points [L, N, 3]; with `pose` [L, 6] one trans [4, 4], else per-frame trans
+    [L, 4, 4]. Returns fp64 [L, N, 2] pixel coordinates of a width x height image."""
+    points = _float_operand(points, "project_points: points", lambda s: len(s) == 3 and s[0] > 0 and s[1] > 0 and s[2] == 3)
+    L = points.shape[0]
+    if pose is None:
+        trans = _float_operand(trans, "project_points: trans", lambda s: tuple(s) == (L, 4, 4))
+    else:
+        trans = _float_operand(trans, "project_points: trans", lambda s: tuple(s) == (4, 4))
+        pose = _float_operand(pose, "project_points: pose", lambda s: len(s) == 2 and s[0] >= L and s[1] == 6)
+    out = torch.empty(L, points.shape[1], 2, dtype=torch.float64, device=points.device)
+    f64 = lambda t: I(t is not None and t.dtype == torch.float64)  # noqa: E731
+    check(lib().ap_project_points(ptr(points), f64(points), I(L), I(points.shape[1]), ptr(trans), f64(trans), ptr(pose),
+                                  f64(pose), I(int(width)), I(int(height)), ptr(out), stream_ptr()), "ap_project_points")
+    _count()
+    return out
+
+
+def facemesh_raster(keypoints: torch.Tensor, edges: torch.Tensor, colours: torch.Tensor, width: int, height: int,
+                    normed: bool = False) -> torch.Tensor:
+    """Face-mesh pose maps: keypoints [L, N, 2] (fp32 / fp64; pixels of a width x height image, or normalised) drawn as
+    thickness-2 cv2 lines of `edges` (int32 [E, 3]: a, b, colour group) in `colours` (uint8 [G, 3]) on a 512 x 512
+    canvas, resized to width x height (multiples of 8). Returns uint8 [L, height, width, 3]."""
+    keypoints = _float_operand(keypoints, "facemesh_raster: keypoints",
+                               lambda s: len(s) == 3 and s[0] > 0 and s[1] > 0 and s[2] == 2)
+    _ensure(edges)
+    _ensure(colours)
+    if edges.dtype != torch.int32 or edges.dim() != 2 or edges.shape[1] != 3 or not edges.is_contiguous():
+        raise ValueError("facemesh_raster: edges must be contiguous int32 [E, 3]")
+    if colours.dtype != torch.uint8 or colours.dim() != 2 or colours.shape[1] != 3 or not colours.is_contiguous():
+        raise ValueError("facemesh_raster: colours must be contiguous uint8 [G, 3]")
+    W, H = int(width), int(height)
+    if W <= 0 or H <= 0 or W % 8 or H % 8:
+        raise ValueError(f"facemesh_raster: width {W} and height {H} must be positive multiples of 8")
+    L, N = keypoints.shape[:2]
+    canvas = torch.empty(L, 512, 512, dtype=torch.uint8, device=keypoints.device)
+    out = torch.empty(L, H, W, 3, dtype=torch.uint8, device=keypoints.device)
+    check(lib().ap_facemesh_raster(ptr(keypoints), I(keypoints.dtype == torch.float64), I(L), I(N), I(bool(normed)), I(W),
+                                   I(H), ptr(edges), I(edges.shape[0]), ptr(colours), I(colours.shape[0]), ptr(canvas),
+                                   ptr(out), stream_ptr()), "ap_facemesh_raster")
+    _count(2)
+    return out

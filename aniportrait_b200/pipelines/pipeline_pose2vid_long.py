@@ -175,7 +175,14 @@ class Pose2VideoPipeline:
     def _pose_maps_to_tensor(self, pose_images, height, width, device):
         """cond_image_processor.preprocess for the pose maps. uint8 HxWx3 arrays of the target size (what the scripts
         pass, pose2vid.py:153-158) take a fast path: the bytes go to the GPU and the reference's `2*x - 1` (no /255, see
-        image_processor.py) is evaluated there in fp32 — identical values, 4x fewer bytes over PCIe, no host float pass."""
+        image_processor.py) is evaluated there in fp32 — identical values, 4x fewer bytes over PCIe, no host float pass.
+        A CUDA uint8 tensor [L, H, W, 3] of the target size (the pose maps of audio_models.audio_to_pose_maps) takes the
+        same path without the host copy."""
+        if isinstance(pose_images, torch.Tensor) and pose_images.is_cuda and pose_images.dtype == torch.uint8:
+            if pose_images.dim() != 4 or tuple(pose_images.shape[1:]) != (height, width, 3):
+                raise ValueError(f"pose_images: a CUDA uint8 tensor must be [L, {height}, {width}, 3], "
+                                 f"got {tuple(pose_images.shape)}")
+            return pose_images.to(device).permute(0, 3, 1, 2).to(torch.float32) * 2.0 - 1.0
         frames = list(pose_images)
         if all(isinstance(p, np.ndarray) and p.dtype == np.uint8 and p.ndim == 3 and p.shape[:2] == (height, width)
                for p in frames):

@@ -263,6 +263,37 @@ int ap_pos_conv_gelu_f16(const void* x, int T, const void* w, const float* bias,
  */
 int ap_mean_f16(const void* x, int n_src, long long n, float* out_f32, void* out_f16, void* stream);
 
+/*
+ * Face-mesh pose maps (audio2vid / vid2vid conditioning; reference src/utils/pose_util.py, src/utils/draw_util.py).
+ *
+ * ap_pose_smooth: smooth_pose_seq(x, window) (pose_util.py:81-88) on x [L, 6], fp32 (f64 = 0) or fp64 (f64 = 1), out the
+ * same dtype: out[i] = mean of rows max(0, i - window/2) .. min(L, i + window/2 + 1) - 1, summed row after row in the
+ * input dtype and divided by the count, without FMA contraction: bit-identical to numpy. out must not alias x.
+ */
+int ap_pose_smooth(const void* x, int L, int window, int f64, void* out, void* stream);
+
+/*
+ * ap_project_points: project_points / project_points_with_trans (pose_util.py:30-59) in fp64. points [L, N, 3] (fp32 or
+ * fp64 per points_f64); `pose` [L, 6] (xyz Euler degrees, extrinsic, then a translation) with one 4 x 4 `trans`, or
+ * pose = NULL with per-frame `trans` [L, 4, 4]; out fp64 [L, N, 2] pixel coordinates of a W x H image, through
+ * create_perspective_matrix(W / H) (63 degree vertical FOV, near 1, far 10000, y flipped, fp32 entries).
+ */
+int ap_project_points(const void* points, int points_f64, int L, int N, const void* trans, int trans_f64, const void* pose,
+                      int pose_f64, int W, int H, double* out, void* stream);
+
+/*
+ * ap_facemesh_raster: FaceMeshVisualizer.draw_landmarks (draw_util.py:124-148) for L frames. keypoints [L, N, 2] (fp32 or
+ * fp64 per kp_f64): pixel coordinates of a W x H image (normed = 0) or normalised ones (normed = 1). Each landmark is
+ * normalised, rounded to fp32, valid iff both coordinates lie in [0, 1], and placed at pixel min(floor(v * 512), 511) of
+ * a 512 x 512 canvas. Every edge e of `edges` (int32 [E, 3]: landmark a, landmark b, colour group g; a, b < N) whose two
+ * landmarks are valid is drawn as cv2.line(thickness=2, LINE_8); a pixel takes the colour of the highest group that
+ * covers it, colours[g] (uint8 [G, 3], written as given: BGR in the reference). The canvas is then resized to W x H as
+ * cv2.resize(INTER_LINEAR) does (W, H multiples of 8). canvas: uint8 workspace [L, 512, 512], 16-byte aligned; out: uint8
+ * [L, H, W, 3]. Deterministic: two calls give the same bytes.
+ */
+int ap_facemesh_raster(const void* keypoints, int kp_f64, int L, int N, int normed, int W, int H, const int* edges, int E,
+                       const unsigned char* colours, int G, void* canvas, void* out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
